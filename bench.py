@@ -5,6 +5,8 @@
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU implementation of the same path
                                                              # (the pinned CPU restatement, oracle/; /root/reference does
                                                              #  not exist on the GPU box)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's samples to DIR/sample.npy,
+                                                             # to compare two builds output for output
 
 One "step" is one iteration of `p_sample_loop` over one batch of 64 motions: one denoiser pass (8-layer MDM
 transformer over 64 x 197 tokens) + the posterior/noise update -- everything the reference does in one loop
@@ -42,6 +44,7 @@ sys.path.insert(0, ROOT)
 
 B, D, L, S, T = 64, 263, 196, 197, 1000
 D_MODEL, FF, LAYERS, HEADS = 512, 1024, 8, 4
+DUMP_LIMIT_BYTES = 64 << 20
 METRIC = "denoising steps/sec (B=64, L=196, D=263, 1000 steps)"
 WORKLOAD = "configs[1]: unconditional DDPM p_sample_loop, T=1000, B=64 per GPU, L=196, D=263, MDM 8L/512d/ff1024/4h"
 MIN_WARMUP = 3
@@ -270,16 +273,30 @@ def cpu_reference_steps(max_steps: int, budget_s: float, warmup: int = 1):
     with torch.no_grad():
         for _ in range(warmup):
             x = O.p_sample(sd, tab, x, torch.full((B,), t_idx), c, noise)["sample"]
-            t_idx -= 1
+            t_idx = (t_idx - 1) % T  # past t = 0 the walk starts over at t = T - 1
         done, t0 = 0, time.perf_counter()
         while done < max_steps:
             x = O.p_sample(sd, tab, x, torch.full((B,), t_idx), c, noise)["sample"]
-            t_idx -= 1
+            t_idx = (t_idx - 1) % T
             done += 1
             if time.perf_counter() - t0 > budget_s:
                 break
         dt = time.perf_counter() - t0
-    return done, dt, threads
+    return done, dt, threads, x
+
+
+def dump_outputs(path: str, arrays: dict):
+    """Write each array as <path>/<name>.npy in float32.  An output larger than DUMP_LIMIT_BYTES keeps a fixed, seeded
+    choice of its motions (rows of dim 0), in their original order."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().to("cpu", torch.float32)
+        rows = DUMP_LIMIT_BYTES // (a[0].numel() * 4)
+        if a.shape[0] > rows:
+            a = a[torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values]
+        np.save(os.path.join(path, f"{name}.npy"), a.numpy())
 
 
 def run_reference(args):
@@ -287,7 +304,9 @@ def run_reference(args):
     if rank != 0:
         return  # the CPU arm runs on rank 0 only
     warm = max(args.warmup, MIN_WARMUP)
-    done, dt, threads = cpu_reference_steps(args.steps, budget_s=150.0, warmup=warm)
+    done, dt, threads, x = cpu_reference_steps(args.steps, budget_s=float("inf"), warmup=warm)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sample": x})
     value = done / dt
     sample = f"{done} consecutive DDPM steps (t={T - 1 - warm}..) of the B=64 unconditional loop on the host CPU, fp32, {threads} threads"
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": done,
@@ -465,10 +484,13 @@ def run_engine(args):
     barrier()
     w0 = time.time()
     e0.record()
-    loop(args.steps)
+    out = loop(args.steps)
     e1.record()
     barrier()
     clocks.window("timed", w0, time.time())
+    if args.dump_outputs and rank == 0:
+        # what the timed loop hands its caller: this rank's samples, or every rank's after the all-gather
+        dump_outputs(args.dump_outputs, {"sample": gathered if world > 1 else out})
     ms = e0.elapsed_time(e1)
     launches = eng.launch_count - launches0
     tms = torch.tensor([ms], device=dev, dtype=torch.float64)
@@ -548,7 +570,7 @@ def run_engine(args):
     # ---- CPU baseline on this box's host cores: a bounded sample of the same workload ----
     cpu = None  # timed at N=1 only (the other ranks' processes would compete for the same host cores)
     if world == 1:
-        done, dt, threads = cpu_reference_steps(max_steps=12, budget_s=25.0)
+        done, dt, threads, _ = cpu_reference_steps(max_steps=12, budget_s=25.0)
         cpu = {"value": done / dt, "unit": UNIT, "cores": threads, "kind": "port",
                "sample": f"{done} consecutive DDPM steps of the same B=64 loop on the host CPU (fp32 PyTorch restatement of the reference)"}
 
@@ -579,7 +601,11 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--precision", default="bf16x3", choices=["bf16x3", "bf16"])
     ap.add_argument("--skip-configs", action="store_true", help="only configs[1]: skip the configs block and the eager-PyTorch baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the samples of the last timed step as DIR/sample.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

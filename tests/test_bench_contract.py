@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import torch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -21,9 +24,9 @@ def _load_bench():
     return mod
 
 
-def test_reference_arm_prints_exactly_one_json_line():
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
-                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+def test_reference_arm_prints_exactly_one_json_line(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, r.stdout
@@ -34,6 +37,20 @@ def test_reference_arm_prints_exactly_one_json_line():
     assert d["impl"] == "reference" and d["higher_is_better"] is True and d["value"] > 0
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
+    assert d["steps"] == 1
+    out = np.load(tmp_path / "sample.npy")
+    assert out.dtype == np.float32 and out.shape == (64, 263, 1, 196) and np.isfinite(out).all()
+
+
+def test_dump_outputs_keeps_a_fixed_choice_of_rows_under_the_size_limit(tmp_path):
+    b = _load_bench()
+    rows = torch.arange(520, dtype=torch.float32)[:, None].expand(520, 32768)   # 128 KiB a row, 65 MiB in all
+    b.dump_outputs(str(tmp_path / "a"), {"sample": rows})
+    b.dump_outputs(str(tmp_path / "b"), {"sample": rows})
+    a, again = np.load(tmp_path / "a" / "sample.npy"), np.load(tmp_path / "b" / "sample.npy")
+    assert a.nbytes <= b.DUMP_LIMIT_BYTES and a.shape == (512, 32768) and np.array_equal(a, again)
+    kept = a[:, 0]
+    assert (np.diff(kept) > 0).all() and (a == kept[:, None]).all()
 
 
 def test_flop_model_matches_the_survey():
