@@ -49,7 +49,7 @@ __device__ __forceinline__ void named_barrier_sync(int id, int nthreads) {
 // are in tensor memory -- the P V product over those keys starts while the remaining probabilities are computed.
 template <int CHUNK0, int NCHUNKS, int EARLY>
 __device__ __forceinline__ float softmax_half(uint32_t trow, int S, bool split, float c_scale, float (*red_max)[128], int half,
-                                              int row, bool trunc, uint32_t col_plo, uint64_t* part_a, int lane) {
+                                              int row, uint32_t col_plo, uint64_t* part_a, int lane) {
   float s[NCHUNKS * 16];
   {
     // all TMEM reads in flight at once, one wait
@@ -82,7 +82,7 @@ __device__ __forceinline__ float softmax_half(uint32_t trow, int S, bool split, 
       const float p0 = fast_exp2(fmaf(s[c * 16 + j * 2], c_scale, -mc));
       const float p1 = fast_exp2(fmaf(s[c * 16 + j * 2 + 1], c_scale, -mc));
       sum += p0 + p1;
-      if (trunc) split_bf16x2_trunc(p0, p1, ph[j], pl[j]); else split_bf16x2(p0, p1, ph[j], pl[j]);
+      split_bf16x2(p0, p1, ph[j], pl[j]);
     }
     tmem_st8(trow + kColPHi + (CHUNK0 + c) * 8, ph);
     if (split) tmem_st8(trow + col_plo + (CHUNK0 + c) * 8, pl);
@@ -355,13 +355,8 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid
       uint32_t hw[32], lw[32];
 #pragma unroll
       for (int j = 0; j < 16; ++j) {
-        if (p.trunc_split) {
-          split_bf16x2_trunc(__uint_as_float(v0[2 * j]) * inv, __uint_as_float(v0[2 * j + 1]) * inv, hw[j], lw[j]);
-          split_bf16x2_trunc(__uint_as_float(v1[2 * j]) * inv, __uint_as_float(v1[2 * j + 1]) * inv, hw[16 + j], lw[16 + j]);
-        } else {
-          split_bf16x2(__uint_as_float(v0[2 * j]) * inv, __uint_as_float(v0[2 * j + 1]) * inv, hw[j], lw[j]);
-          split_bf16x2(__uint_as_float(v1[2 * j]) * inv, __uint_as_float(v1[2 * j + 1]) * inv, hw[16 + j], lw[16 + j]);
-        }
+        split_bf16x2(__uint_as_float(v0[2 * j]) * inv, __uint_as_float(v0[2 * j + 1]) * inv, hw[j], lw[j]);
+        split_bf16x2(__uint_as_float(v1[2 * j]) * inv, __uint_as_float(v1[2 * j + 1]) * inv, hw[16 + j], lw[16 + j]);
       }
       if (group_row0 + 32 <= S) {
         store_block_tma(stage, lane, hw, &map_o_hi, head * kHeadDim + half * 64, row0 + group_row0);
@@ -397,9 +392,9 @@ attention_pair_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid
       tc_fence_after();
       float sum;
       if (half == 0) {
-        sum = softmax_half<0, kChunks0, kEarly0>(trow, S, split, c_scale, bars->red_max, 0, row, p.trunc_split != 0, kPColPLo, &bars->p_part, lane);
+        sum = softmax_half<0, kChunks0, kEarly0>(trow, S, split, c_scale, bars->red_max, 0, row, kPColPLo, &bars->p_part, lane);
       } else {
-        sum = softmax_half<kChunks0, kChunks1, kEarly1>(trow, S, split, c_scale, bars->red_max, 1, row, p.trunc_split != 0, kPColPLo, &bars->p_part, lane);
+        sum = softmax_half<kChunks0, kChunks1, kEarly1>(trow, S, split, c_scale, bars->red_max, 1, row, kPColPLo, &bars->p_part, lane);
       }
       bars->red_sum[half][row] = sum;
       tmem_st_wait();

@@ -73,7 +73,6 @@ extern "C" int cmdi_test_linear(const float* A, const float* W, const float* bia
   if (make_tmap_2d(&mc_f32, C, 4, M, N, N, 32, 32)) return 1;
   LinearStoreMaps stm;
   stm.f32 = &mc_f32;
-  const LinearStoreMaps* stp = getenv("CMDI_EPI") && !strcmp(getenv("CMDI_EPI"), "stg") ? nullptr : &stm;
   LinearParams p{};
   p.M = M; p.N = N; p.K = K; p.nsplit = precision;
   p.bias = bias; p.residual = residual; p.ld_res = N;
@@ -112,9 +111,9 @@ extern "C" int cmdi_test_linear(const float* A, const float* W, const float* bia
       p.out_lo = o_lo.as<__nv_bfloat16>();
       p.ld_bf = Np;
       if (getenv("CMDI_TEST_NOF32")) p.out_f32 = nullptr;
-      CK(launch_linear_pair(ma_hi, ma_lo, mw_hi, mw_lo, p, block_n, num_sms_of_current_device(), stream, stp));
+      CK(launch_linear_pair(ma_hi, ma_lo, mw_hi, mw_lo, p, block_n, num_sms_of_current_device(), stream, &stm));
     }
-    CK(launch_linear_pair(ma_hi, ma_lo, mw_hi, mw_lo, p, block_n, num_sms_of_current_device(), stream, stp));
+    CK(launch_linear_pair(ma_hi, ma_lo, mw_hi, mw_lo, p, block_n, num_sms_of_current_device(), stream, &stm));
     if (want_dbg) {
       std::vector<long long> h(148 * 16);
       CK(cudaStreamSynchronize(stream));
@@ -174,7 +173,6 @@ extern "C" int cmdi_test_attention(const float* qkv, float* O, int num_seqs, int
   AttnParams p{};
   p.num_seqs = num_seqs; p.seq_len = S; p.num_heads = H; p.nsplit = precision; p.nsplit_out = 3;
   p.out_hi = o_hi.as<__nv_bfloat16>(); p.out_lo = o_lo.as<__nv_bfloat16>(); p.ld_out = ldo;
-  if (const char* g = getenv("CMDI_ATTN_SPLIT")) p.trunc_split = strcmp(g, "trunc") == 0;
   DevBuf adbg;
   const int nctas = ((S + 127) / 128) * H * num_seqs;
   if (getenv("CMDI_TEST_DBG")) {

@@ -56,16 +56,6 @@ __device__ __forceinline__ float ln_apply(float x, float mean, float rstd, float
   return __fmaf_rn(__fmul_rn(__fsub_rn(x, mean), rstd), g, b);
 }
 
-// Same split with the hi half taken by truncation (one PRMT instead of a conversion): v = hi + lo still holds to
-// 2^-16 |v| (hi is exact in bf16, lo = RN(v - hi) with |v - hi| < 2^-7 |v|).  Halves the work on the conversion pipe
-// where the values are produced at MUFU rate anyway (softmax probabilities, attention outputs).
-__device__ __forceinline__ void split_bf16x2_trunc(float a, float b, uint32_t& hi_word, uint32_t& lo_word) {
-  const uint32_t ua = __float_as_uint(a), ub = __float_as_uint(b);
-  hi_word = __byte_perm(ua, ub, 0x7632);
-  const __nv_bfloat162 l = __floats2bfloat162_rn(a - __uint_as_float(ua & 0xffff0000u), b - __uint_as_float(ub & 0xffff0000u));
-  lo_word = *reinterpret_cast<const uint32_t*>(&l);
-}
-
 // ----------------------------------------------------------------------------------------------
 // programmatic dependent launch: a kernel launched with programmaticStreamSerializationAllowed may start while its
 // predecessor drains; it must not touch global memory before griddep_wait() (no-op for ordinary launches)

@@ -3,10 +3,14 @@
 // One engine per device.  It owns (a) the MDM weights as bf16 hi/lo planes + their TMA descriptors,
 // (b) the diffusion tables as fp32 device arrays, (c) every activation buffer of one denoiser pass, sized
 // once for 2*max_batch sequences (the CFG cond+uncond pass is one batch-doubled pass), and (d) one captured
-// CUDA graph per loop configuration.  A sampling step is 60 kernel launches of this library and nothing else:
+// CUDA graph per loop configuration.  A sampling step is 20 kernel launches of this library (plus one memset of the
+// chain's dependency counters) and nothing else:
 //
-//   token_rows -> frame-embed GEMM -> 8 x [QKV GEMM, attention, out-proj GEMM(+residual), LayerNorm,
-//                 FFN1 GEMM(+GELU), FFN2 GEMM(+residual), LayerNorm] -> output-head GEMM -> diffusion_step
+//   token_rows -> frame-embed GEMM -> QKV_0 GEMM -> 8 x [attention, chain: out-proj(+residual), FFN1(+GELU),
+//                 FFN2(+residual), QKV_{l+1} | output head] -> diffusion_step
+//
+// with every LayerNorm folded into the GEMMs around it (run_denoiser_chain).  Guided steps and CMDI_CHAIN=0 run the
+// unchained pass instead: one launch per linear layer plus the LayerNorm kernels, 60 launches per step.
 //
 // The step index lives on the device (decremented by diffusion_step), so the same graph is replayed for
 // every step of a loop with no host work in between (reference: one Python iteration + ~150 PyTorch ops
@@ -85,11 +89,11 @@ struct ChainTables {  // per number of sequences: the phase lists of the chained
   int num_phases = 4;
 };
 
-struct GraphKey {
+struct GraphKey {  // compared with memcmp: no padding bytes
   int B, cfg, sampler, impute, stop_at, tape_mode, has_cond;
   float eta;
   const void* tape;
-  int t0, uncond, guided, group;
+  int uncond, guided;
   bool operator<(const GraphKey& o) const { return memcmp(this, &o, sizeof(GraphKey)) < 0; }
 };
 
@@ -99,13 +103,9 @@ struct cmdi_engine {
   cmdi_model_cfg cfg{};
   int device = 0, num_sms = 148;
   int nsplit = 3;
-  int bn_qkv = kBnWide;
-  int debug = 0, bn_wide = kBnWide, bn_narrow = kBnNarrow;  // CMDI_DEBUG / CMDI_BN_WIDE / CMDI_BN_NARROW (bring-up knobs)
-  int steps_per_graph = 1;  // CMDI_GRAPH_STEPS: consecutive steps captured into one graph (10 and 50 measured: no gain over 1)
+  int debug = 0;            // CMDI_DEBUG (bring-up knob)
   bool no_graph = false;    // CMDI_NO_GRAPH=1: plain stream launches even when the caller asks for graph replay
-  int attn_trunc_split = 0;  // CMDI_ATTN_SPLIT=trunc
   float2 *ln_stats1 = nullptr, *ln_stats2 = nullptr;  // (mean, rstd) per token row published by norm1 / norm2
-  bool tma_store = true;  // CMDI_EPI=stg selects the coalesced-STG epilogue everywhere
   int D = 263, D_pad = 264, L = 196, S = 197, ff = 1024, H = 4, layers = 8, maxB = 0;
   int max_seqs = 0, seq_rows = 0, seq_rows_pad = 0, frame_rows = 0, frame_rows_pad = 0;
   std::vector<void*> allocs;
@@ -134,7 +134,7 @@ struct cmdi_engine {
   Planes xseq_p, x1_p, qkv_p, attn_p, ffh_p;
   CUtensorMap q_map_hi{}, q_map_lo{}, kv_map_hi{}, kv_map_lo{}, kh_map_hi{}, kh_map_lo{};  // Q {64,128}, K/V {64,208}, K half {64,104}
   CUtensorMap vsum_st{};  // fp32 TMA-store target for the pre-LayerNorm sums
-  CUtensorMap xseq_st{}, x1_st{};  // fp32 TMA-store targets: xseq (backward pass), x1 (v1 of the chained forward path)
+  CUtensorMap xseq_st{};  // fp32 TMA-store target of xseq (backward pass)
   uint8_t* obs_mask = nullptr;
   float *cond_emb = nullptr, *cond_proj = nullptr, *text_scale = nullptr;
   int* step_ctr = nullptr;  // [2]: step index, block-arrival counter
@@ -156,9 +156,6 @@ struct cmdi_engine {
   // which guided steps (they stash LayerNorm inputs for the backward pass) always use.
   bool use_chain = true;
   int chain_skip = 0;         // CMDI_CHAIN_SKIP=4 / 2: timing decomposition without operand loads / without MMAs (wrong results)
-  int chain_res_planes = 1;   // CMDI_CHAIN_RES=f32: residual sources kept as fp32 copies (A/B)
-  int chain_wide = 1;         // CMDI_CHAIN_WIDE=0: 32-column slices in the planes-only phases too (A/B)
-  int chain_publish_now = 1;  // CMDI_CHAIN_PUBLISH=deferred: counter bumps deferred to the warp's next tile
   std::vector<FoldedW> f_qkv, f_w1;
   FoldedW f_out;
   std::vector<float*> beta_bo, beta_b2;         // [layer]: norm2_{l-1}.bias + out_proj_l.bias, norm1_l.bias + linear2_l.bias (chained epilogues)
@@ -262,10 +259,8 @@ int run_linear(cmdi_engine* e, const Planes& a, const Planes& w, const LinearPar
   LinearParams p = p_in;
   p.debug = e->debug;
   LinearStoreMaps st;
-  if (e->tma_store) {
-    if (out_planes) { st.hi = &out_planes->st_hi; st.lo = &out_planes->st_lo; }
-    st.f32 = out_f32;
-  }
+  if (out_planes) { st.hi = &out_planes->st_hi; st.lo = &out_planes->st_lo; }
+  st.f32 = out_f32;
   if (a.has_tap) { st.a_tap_hi = &a.tap_hi; st.a_tap_lo = &a.tap_lo; }
   CK(launch_linear_pair(a.map_hi, a.map_lo, w.pair_hi, w.pair_lo, p, block_n, e->num_sms, s, &st));
   return 0;
@@ -326,12 +321,12 @@ int run_denoiser(cmdi_engine* e, int B, bool dup, int n_cond_seqs, bool has_cond
     LinearParams q{};
     q.M = M; q.N = 3 * kDModel; q.K = kDModel; q.nsplit = e->nsplit; q.bias = w.bqkv;
     q.out_hi = qkv_out.hi; q.out_lo = qkv_out.lo; q.ld_bf = 3 * kDModel; q.nsplit_out = e->nsplit;
-    for (int r_ = 0; r_ < reps; ++r_) CKI(run_linear(e, e->xseq_p, w.wqkv, q, e->bn_qkv, s, &qkv_out));
+    for (int r_ = 0; r_ < reps; ++r_) CKI(run_linear(e, e->xseq_p, w.wqkv, q, kBnWide, s, &qkv_out));
     CKI(mark());
     // attention core
     AttnParams a{};
     a.num_seqs = nseq; a.seq_len = e->S; a.num_heads = e->H; a.nsplit = e->nsplit; a.nsplit_out = e->nsplit;
-    a.out_hi = e->attn_p.hi; a.out_lo = e->attn_p.lo; a.ld_out = kDModel; a.trunc_split = e->attn_trunc_split;
+    a.out_hi = e->attn_p.hi; a.out_lo = e->attn_p.lo; a.ld_out = kDModel;
     const AttnMaps am = ls ? AttnMaps{&ls->q_hi, &ls->q_lo, &ls->kh_hi, &ls->kh_lo, &ls->kv_hi, &ls->kv_lo, &e->attn_p.st_hi, &e->attn_p.st_lo}
                            : AttnMaps{&e->q_map_hi, &e->q_map_lo, &e->kh_map_hi, &e->kh_map_lo, &e->kv_map_hi, &e->kv_map_lo, &e->attn_p.st_hi, &e->attn_p.st_lo};
     for (int r_ = 0; r_ < reps; ++r_) CK(launch_attention(am, a, s));
@@ -380,7 +375,7 @@ int run_denoiser(cmdi_engine* e, int B, bool dup, int n_cond_seqs, bool has_cond
   return 0;
 }
 bool chain_eligible(const cmdi_engine* e) {
-  return e->use_chain && e->tma_store && e->debug == 0 && e->layers >= 1;
+  return e->use_chain && e->debug == 0 && e->layers >= 1;
 }
 
 // Phase lists for `nseq` sequences: layer l = [out-proj_l, FFN1_l, FFN2_l, QKV_{l+1} | output head].
@@ -398,17 +393,17 @@ int get_chain_tables(cmdi_engine* e, int nseq, const ChainTables** out) {
   auto base = [&](ChainPhaseDesc& d, const Planes& a, const CUtensorMap& w_hi, const CUtensorMap& w_lo, int N, int K, int bn) {
     memset(&d, 0, sizeof(d));
     d.a_hi = a.map_hi; d.a_lo = a.map_lo; d.w_hi = w_hi; d.w_lo = w_lo;
-    d.o_hi = a.map_hi; d.o_lo = a.map_hi; d.o_f32 = a.map_hi;  // placeholders unless set below
+    d.o_hi = a.map_hi; d.o_lo = a.map_hi;  // placeholders unless set below
     ChainPhaseInfo& pi = d.info;
     pi.p.M = M; pi.p.N = N; pi.p.K = K; pi.p.nsplit = e->nsplit; pi.p.nsplit_out = e->nsplit; pi.p.rowmap = ROWMAP_IDENTITY;
-    pi.p.tma_store = 1; pi.p.debug = e->chain_skip;
+    pi.p.debug = e->chain_skip;
     pi.block_n = bn; pi.num_m_pairs = m_pairs; pi.num_n_blocks = (N + bn - 1) / bn; pi.num_k_blocks = (K + 63) / 64;
   };
   for (int l = 0; l < e->layers; ++l) {
     const LayerW& w = e->lw[l];
     ChainPhaseDesc* ph = &host[(size_t)l * kMaxChainPhases];
     int* ctr = e->chain_ctr + (size_t)l * 3 * e->max_m_pairs;
-    // out-proj + residual -> v1 (fp32 + planes + partial statistics)
+    // out-proj + residual -> v1 (planes + partial statistics)
     base(ph[0], e->attn_p, e->wo_chain[2 * l], e->wo_chain[2 * l + 1], kDModel, kDModel, kBnWide);
     {
       LinearParams& p = ph[0].info.p;
@@ -416,13 +411,10 @@ int get_chain_tables(cmdi_engine* e, int nseq, const ChainTables** out) {
       else {
         // bias folded into the beta of the re-derived LayerNorm residual: one vector (and 32 shuffles + adds per slice) less
         p.ld_ln = kDModel; p.ln_partials = e->stats2; p.ln_gamma = e->lw[l - 1].g2; p.ln_beta = e->beta_bo[l];
-        if (e->chain_res_planes) { p.ln_src_hi = e->xseq_p.hi; p.ln_src_lo = e->xseq_p.lo; }
-        else p.ln_src = e->vsum;
+        p.ln_src_hi = e->xseq_p.hi; p.ln_src_lo = e->xseq_p.lo;
       }
-      // the fp32 copy of v1 is only ever read back as FFN2's residual source: not written when that reads the planes
-      if (!e->chain_res_planes) { p.out_f32 = e->x1; p.ld_f32 = kDModel; }
       p.out_hi = e->x1_p.hi; p.out_lo = e->x1_p.lo; p.ld_bf = kDModel; p.stats_out = e->stats1;
-      ph[0].o_hi = e->x1_p.st32_hi; ph[0].o_lo = e->x1_p.st32_lo; ph[0].o_f32 = e->x1_st;
+      ph[0].o_hi = e->x1_p.st32_hi; ph[0].o_lo = e->x1_p.st32_lo;
       ph[0].info.done_ctr = ctr;
     }
     // FFN1 (norm1 folded) + GELU -> hidden planes
@@ -431,20 +423,18 @@ int get_chain_tables(cmdi_engine* e, int nseq, const ChainTables** out) {
       LinearParams& p = ph[1].info.p;
       p.bias = e->f_w1[l].d; p.fold_c = e->f_w1[l].c; p.fold_stats = e->stats1; p.act = 1;
       p.out_hi = e->ffh_p.hi; p.out_lo = e->ffh_p.lo; p.ld_bf = e->ff;
-      if (e->chain_wide) { ph[1].info.wide = 1; ph[1].o_hi = e->ffh_p.st_hi; ph[1].o_lo = e->ffh_p.st_lo; }
-      else { ph[1].o_hi = e->ffh_p.st32_hi; ph[1].o_lo = e->ffh_p.st32_lo; }
+      ph[1].info.pair_epilogue = 1; ph[1].o_hi = e->ffh_p.st_hi; ph[1].o_lo = e->ffh_p.st_lo;
       ph[1].info.wait_ctr = ctr; ph[1].info.wait_target = ph[0].info.num_n_blocks * 2;
       ph[1].info.done_ctr = ctr + e->max_m_pairs;
     }
-    // FFN2 + residual LN1(v1) -> v2 (fp32 + planes + partial statistics)
+    // FFN2 + residual LN1(v1) -> v2 (planes + partial statistics)
     base(ph[2], e->ffh_p, e->w2_chain[2 * l], e->w2_chain[2 * l + 1], kDModel, e->ff, kBnWide);
     {
       LinearParams& p = ph[2].info.p;
       p.ld_ln = kDModel; p.ln_partials = e->stats1; p.ln_gamma = w.g1; p.ln_beta = e->beta_b2[l];
-      if (e->chain_res_planes) { p.ln_src_hi = e->x1_p.hi; p.ln_src_lo = e->x1_p.lo; }
-      else { p.ln_src = e->x1; p.out_f32 = e->vsum; p.ld_f32 = kDModel; }
+      p.ln_src_hi = e->x1_p.hi; p.ln_src_lo = e->x1_p.lo;
       p.out_hi = e->xseq_p.hi; p.out_lo = e->xseq_p.lo; p.ld_bf = kDModel; p.stats_out = e->stats2;
-      ph[2].o_hi = e->xseq_p.st32_hi; ph[2].o_lo = e->xseq_p.st32_lo; ph[2].o_f32 = e->vsum_st;
+      ph[2].o_hi = e->xseq_p.st32_hi; ph[2].o_lo = e->xseq_p.st32_lo;
       ph[2].info.wait_ctr = ctr + e->max_m_pairs; ph[2].info.wait_target = ph[1].info.num_n_blocks * 2;
       ph[2].info.done_ctr = ctr + 2 * e->max_m_pairs;
     }
@@ -455,19 +445,17 @@ int get_chain_tables(cmdi_engine* e, int nseq, const ChainTables** out) {
       LinearParams& p = ph[3].info.p;
       p.bias = fq.d; p.fold_c = fq.c; p.fold_stats = e->stats2;
       p.out_hi = e->qkv_p.hi; p.out_lo = e->qkv_p.lo; p.ld_bf = 3 * kDModel;
-      if (e->chain_wide) { ph[3].info.wide = 1; ph[3].o_hi = e->qkv_p.st_hi; ph[3].o_lo = e->qkv_p.st_lo; }
-      else { ph[3].o_hi = e->qkv_p.st32_hi; ph[3].o_lo = e->qkv_p.st32_lo; }
+      ph[3].info.pair_epilogue = 1; ph[3].o_hi = e->qkv_p.st_hi; ph[3].o_lo = e->qkv_p.st_lo;
     } else {
       // output head on tokens 1.. (norm2 of the last layer folded), frame-major fp32 rows
       base(ph[3], e->xseq_p, e->f_out.w.pair_hi, e->f_out.w.pair_lo, e->D_pad, kDModel, kBnWide);
       LinearParams& p = ph[3].info.p;
       p.bias = e->f_out.d; p.fold_c = e->f_out.c; p.fold_stats = e->stats2;
-      p.rowmap = ROWMAP_SEQ_TO_FRAMES; p.frames = e->L; p.out_f32 = e->model_out; p.ld_f32 = e->D_pad; p.tma_store = 0;
+      p.rowmap = ROWMAP_SEQ_TO_FRAMES; p.frames = e->L; p.out_f32 = e->model_out; p.ld_f32 = e->D_pad;
     }
     ph[3].info.wait_ctr = ctr + 2 * e->max_m_pairs; ph[3].info.wait_target = ph[2].info.num_n_blocks * 2;
     int tiles = 0;
     for (int i = 0; i < kMaxChainPhases; ++i) {
-      ph[i].info.publish_now = e->chain_publish_now;
       ph[i].info.tile_begin = tiles;
       tiles += ph[i].info.num_m_pairs * ph[i].info.num_n_blocks;
       ph[i].info.tile_end = tiles;
@@ -524,11 +512,11 @@ int run_denoiser_chain(cmdi_engine* e, int B, bool dup, int n_cond_seqs, bool ha
   LinearParams q{};
   q.M = M; q.N = 3 * kDModel; q.K = kDModel; q.nsplit = e->nsplit; q.bias = e->lw[0].bqkv;
   q.out_hi = e->qkv_p.hi; q.out_lo = e->qkv_p.lo; q.ld_bf = 3 * kDModel; q.nsplit_out = e->nsplit;
-  for (int r_ = 0; r_ < reps; ++r_) CKI(run_linear(e, e->xseq_p, e->lw[0].wqkv, q, e->bn_qkv, s, &e->qkv_p));
+  for (int r_ = 0; r_ < reps; ++r_) CKI(run_linear(e, e->xseq_p, e->lw[0].wqkv, q, kBnWide, s, &e->qkv_p));
   CKI(mark());
   AttnParams a{};
   a.num_seqs = nseq; a.seq_len = e->S; a.num_heads = e->H; a.nsplit = e->nsplit; a.nsplit_out = e->nsplit;
-  a.out_hi = e->attn_p.hi; a.out_lo = e->attn_p.lo; a.ld_out = kDModel; a.trunc_split = e->attn_trunc_split;
+  a.out_hi = e->attn_p.hi; a.out_lo = e->attn_p.lo; a.ld_out = kDModel;
   const AttnMaps am{&e->q_map_hi, &e->q_map_lo, &e->kh_map_hi, &e->kh_map_lo, &e->kv_map_hi, &e->kv_map_lo, &e->attn_p.st_hi, &e->attn_p.st_lo};
   for (int l = 0; l < e->layers; ++l) {
     for (int r_ = 0; r_ < reps; ++r_)
@@ -698,17 +686,9 @@ extern "C" int cmdi_engine_create(const cmdi_model_cfg* cfg, int device, cmdi_en
   CK(configure_linear_chain_kernel());
   cmdi_engine* e = new cmdi_engine();
   if (const char* g = getenv("CMDI_DEBUG")) e->debug = atoi(g);
-  if (const char* g = getenv("CMDI_EPI")) e->tma_store = strcmp(g, "stg") != 0;
-  e->bn_qkv = kBnWide;  // 256 x 192 pair tiles (CMDI_BN_QKV=192) measured no faster than 256 x 256 despite the better round count
-  if (const char* g = getenv("CMDI_BN_QKV")) e->bn_qkv = atoi(g);
   if (const char* g = getenv("CMDI_NO_GRAPH")) e->no_graph = atoi(g) != 0;
-  if (const char* g = getenv("CMDI_GRAPH_STEPS")) e->steps_per_graph = atoi(g) > 0 ? atoi(g) : 1;
-  if (const char* g = getenv("CMDI_ATTN_SPLIT")) e->attn_trunc_split = strcmp(g, "trunc") == 0;
   if (const char* g = getenv("CMDI_CHAIN")) e->use_chain = atoi(g) != 0;
   if (const char* g = getenv("CMDI_CHAIN_SKIP")) e->chain_skip = atoi(g) & 6;
-  if (const char* g = getenv("CMDI_CHAIN_RES")) e->chain_res_planes = strcmp(g, "f32") != 0;
-  if (const char* g = getenv("CMDI_CHAIN_WIDE")) e->chain_wide = atoi(g) != 0;
-  if (const char* g = getenv("CMDI_CHAIN_PUBLISH")) e->chain_publish_now = strcmp(g, "deferred") != 0;
   e->cfg = *cfg; e->device = device; e->num_sms = prop.multiProcessorCount; e->nsplit = cfg->precision;
   // the chained launches spin on counters other CTA pairs bump: every pair must be resident at once
   if (e->use_chain && linear_chain_max_clusters(e->num_sms) < e->num_sms / 2) e->use_chain = false;
@@ -729,7 +709,7 @@ extern "C" int cmdi_engine_create(const cmdi_model_cfg* cfg, int device, cmdi_en
   A(dev_alloc(e, &e->b_out, round_up(e->D_pad, kBnNarrow)));
   e->lw.resize(e->layers);
   for (auto& w : e->lw) {
-    A(alloc_planes(e, &w.wqkv, 3 * kDModel, kDModel, kDModel, e->bn_qkv));
+    A(alloc_planes(e, &w.wqkv, 3 * kDModel, kDModel, kDModel, kBnWide));
     A(alloc_planes(e, &w.wo, kDModel, kDModel, kDModel, kBnNarrow));
     A(alloc_planes(e, &w.w1, e->ff, kDModel, kDModel, kBnWide));
     A(alloc_planes(e, &w.w2, kDModel, e->ff, e->ff, kBnNarrow));
@@ -776,7 +756,6 @@ extern "C" int cmdi_engine_create(const cmdi_model_cfg* cfg, int device, cmdi_en
   A(make_tmap_bf16_2d(&e->kh_map_lo, e->qkv_p.lo, e->seq_rows_pad, 3 * kDModel, 3 * kDModel, 64, kAttnKeyPad / 2));
   A(make_tmap_2d(&e->vsum_st, e->vsum, 4, e->seq_rows_pad, kDModel, kDModel, 32, 32));
   A(make_tmap_2d(&e->xseq_st, e->xseq, 4, e->seq_rows_pad, kDModel, kDModel, 32, 32));
-  A(make_tmap_2d(&e->x1_st, e->x1, 4, e->seq_rows_pad, kDModel, kDModel, 32, 32));
   A(dev_alloc(e, &e->model_out, (size_t)2 * e->frame_rows_pad * e->D_pad));
   A(dev_alloc(e, &e->pred_x0, (size_t)e->frame_rows_pad * e->D_pad));
   A(dev_alloc(e, &e->x_obs, (size_t)e->frame_rows_pad * e->D_pad));
@@ -1269,13 +1248,13 @@ extern "C" int cmdi_sample(cmdi_engine* e, const cmdi_sample_args* a, float* out
     return 0;
   };
 
-  auto get_exec = [&](bool guided, int group, cudaGraphExec_t* out_exec) -> int {
+  auto get_exec = [&](bool guided, cudaGraphExec_t* out_exec) -> int {
     GraphKey key{};
     memset(&key, 0, sizeof(key));
     key.B = B; key.cfg = a->cfg != 0; key.sampler = a->sampler; key.impute = a->imputate != 0;
     key.stop_at = a->stop_imputation_at; key.tape_mode = tape != nullptr; key.has_cond = has_cond; key.eta = a->eta;
-    key.tape = tape; key.t0 = 0; key.uncond = a->uncond != 0;  // the first step index lives in device memory
-    key.guided = guided; key.group = group;
+    key.tape = tape; key.uncond = a->uncond != 0;  // no first step index: it lives in device memory
+    key.guided = guided;
     auto it = e->graphs.find(key);
     if (it != e->graphs.end()) {
       *out_exec = it->second;
@@ -1286,8 +1265,7 @@ extern "C" int cmdi_sample(cmdi_engine* e, const cmdi_sample_args* a, float* out
     CK(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
     cudaGraph_t graph = nullptr;
     CK(cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal));
-    int erc = 0;
-    for (int g = 0; g < group && !erc; ++g) erc = enqueue_step(cs, guided);
+    const int erc = enqueue_step(cs, guided);
     cudaError_t ce = cudaStreamEndCapture(cs, &graph);
     cudaStreamDestroy(cs);
     if (erc) return 1;
@@ -1303,17 +1281,13 @@ extern "C" int cmdi_sample(cmdi_engine* e, const cmdi_sample_args* a, float* out
     for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second);
     e->graphs.clear();
   }
-  // graphs of `group` consecutive steps (one launch replays that many steps: the per-launch cost of a graph is paid
-  // once per group); single-step graphs serve the remainder and the steps whose pred_xstart is dumped
-  const int group = e->steps_per_graph > 1 ? e->steps_per_graph : 1;
-  cudaGraphExec_t exec1[2] = {nullptr, nullptr}, execg[2] = {nullptr, nullptr};  // [guided]
+  // one graph per step (capturing 10 or 50 consecutive steps into one graph was measured: no gain)
+  cudaGraphExec_t exec[2] = {nullptr, nullptr};  // [guided]
 
   int dump_i = 0;
-  auto guided_at = [&](int k) { return a->recon_guidance && (t0 - k) >= a->stop_recguidance_at; };
-  for (int k = 0; k < nsteps;) {
+  for (int k = 0; k < nsteps; ++k) {
     // utils/editing_util.py:325-333: guidance is active while t >= stop_recguidance_at (t is uniform over the batch)
-    const bool guided = guided_at(k);
-    int run = 1;
+    const bool guided = a->recon_guidance && (t0 - k) >= a->stop_recguidance_at;
     // use_graph 1: calls of one or two steps are launched directly unless a step graph of this configuration already
     // exists (capturing and instantiating one costs more than it saves there); use_graph 2 (the *_progressive
     // generators: one native call per step, many calls): always through the step graph
@@ -1325,25 +1299,17 @@ extern "C" int cmdi_sample(cmdi_engine* e, const cmdi_sample_args* a, float* out
       memset(&probe, 0, sizeof(probe));
       probe.B = B; probe.cfg = a->cfg != 0; probe.sampler = a->sampler; probe.impute = a->imputate != 0;
       probe.stop_at = a->stop_imputation_at; probe.tape_mode = tape != nullptr; probe.has_cond = has_cond; probe.eta = a->eta;
-      probe.tape = tape; probe.uncond = a->uncond != 0; probe.guided = guided; probe.group = 1;
+      probe.tape = tape; probe.uncond = a->uncond != 0; probe.guided = guided;
       via_graph = e->graphs.count(probe) != 0;
     }
     if (via_graph) {
-      const bool dump_in_group = a->dump_xstart && dump_i < a->n_dump && a->dump_steps[dump_i] < k + group;
-      if (group > 1 && k + group <= nsteps && !dump_in_group && guided_at(k + group - 1) == guided) {
-        if (!execg[guided]) CKI(get_exec(guided, group, &execg[guided]));
-        CK(cudaGraphLaunch(execg[guided], s));
-        run = group;
-      } else {
-        if (!exec1[guided]) CKI(get_exec(guided, 1, &exec1[guided]));
-        CK(cudaGraphLaunch(exec1[guided], s));
-      }
+      if (!exec[guided]) CKI(get_exec(guided, &exec[guided]));
+      CK(cudaGraphLaunch(exec[guided], s));
     } else {
       CKI(enqueue_step(s, guided));
     }
-    e->launches += (long long)run * (launches_per_pass(e, guided) + 1 + (guided ? launches_per_backward(e) : 0));
-    k += run;
-    if (a->dump_xstart && dump_i < a->n_dump && a->dump_steps[dump_i] == k - 1) {
+    e->launches += launches_per_pass(e, guided) + 1 + (guided ? launches_per_backward(e) : 0);
+    if (a->dump_xstart && dump_i < a->n_dump && a->dump_steps[dump_i] == k) {
       if (host) {
         CK(launch_frames_to_ref(e->pred_x0, B, e->D, e->L, e->D_pad, e->ref_b, s));
         CK(cudaMemcpyAsync(a->dump_xstart + (size_t)dump_i * n, e->ref_b, n * 4, cudaMemcpyDeviceToHost, s));
@@ -1468,7 +1434,7 @@ extern "C" int cmdi_profile_pass(cmdi_engine* e, int batch, int cfg, int repeats
     CK(cudaMemcpy(h.data(), e->chain_dbg, h.size() * 8, cudaMemcpyDeviceToHost));
     CK(cudaMemset(e->chain_dbg, 0, h.size() * 8));
     const char* names[16] = {"tiles", "tma_dep_wait", "tma_slot_wait", "mma_operand_wait", "mma_acc_wait", "epi0_acc_wait", "epi0_slices", "epi0_publish",
-                             "s_rowstats", "s_stage_free", "s_loads+acc", "s_fold_bias_res", "s_stats_act", "s_f32_store", "s_plane_store", "-"};
+                             "s_rowstats", "s_stage_free", "s_loads+acc", "s_fold_bias_res", "s_stats", "s_f32_store", "s_plane_store", "-"};
     for (int ph = 0; ph < kMaxChainPhases; ++ph) {
       double tiles = 0, acc[16] = {0};
       for (int b = 0; b < e->num_sms; ++b) {

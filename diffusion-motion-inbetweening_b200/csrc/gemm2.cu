@@ -13,7 +13,6 @@
 //   empty[s]      per CTA, signalled by the leader's tcgen05.commit multicast to both CTAs
 //   tmem_full[a]  per CTA, same multicast commit
 //   tmem_empty[a] on the leader: epilogue warps of BOTH CTAs arrive on it (remote arrive from the peer)
-#include <cstdlib>
 #include "common.cuh"
 #include "gemm_epilogue.cuh"
 #include "kernels.h"
@@ -59,9 +58,9 @@ linear2_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
                const LinearParams p, const int num_stages, const int num_m_pairs, const int num_n_blocks) {
   constexpr int kHalfN = BLOCK_N / 2;               // W rows this CTA loads
   constexpr int kBBytes = kHalfN * kBlockK * 2;
-  // double-buffered accumulator: 128 lanes x BLOCK_N fp32 each (allocation rounded up to a power of two)
-  constexpr uint32_t kTmemCols = BLOCK_N == 128 ? 256 : 512;
-  static_assert(BLOCK_N == 128 || BLOCK_N == 192 || BLOCK_N == 256, "BLOCK_N");
+  // double-buffered accumulator: 128 lanes x BLOCK_N fp32 each
+  constexpr uint32_t kTmemCols = 2 * BLOCK_N;
+  static_assert(BLOCK_N == 128 || BLOCK_N == 256, "BLOCK_N");
 
   griddep_launch_dependents();
   extern __shared__ uint8_t smem_raw[];
@@ -354,8 +353,7 @@ cudaError_t launch_impl2(const CUtensorMap& a_hi, const CUtensorMap& a_lo, const
   bool reuse = st && st->a_tap_hi && (nplanes == 1 || st->a_tap_lo) && p.num_taps >= 2 && p.num_taps <= kTapRows - kBlockM + 1;
   for (int t = 1; reuse && t < p.num_taps; ++t)
     reuse = p.tap_a_col[t] == p.tap_a_col[0] && p.tap_row[t] == p.tap_row[0] + t;
-  static const bool reuse_off = getenv("CMDI_CONV_REUSE") && atoi(getenv("CMDI_CONV_REUSE")) == 0;  // bring-up A/B
-  if (reuse && !reuse_off) {
+  if (reuse) {
     const int w_bytes = nplanes * kBBytes, a_bytes = kTapStagesA * nplanes * kATapBytes;
     int num_stages = (kSmemLimit - fixed - a_bytes) / w_bytes;
     if (num_stages > 4) num_stages = 4;  // beyond ~200 KB the L1 left for the epilogue costs more than the depth buys
@@ -378,8 +376,8 @@ cudaError_t configure_linear2_kernels() {
   auto set = [&](auto kernel) {
     if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
   };
-  set(linear2_kernel<128, false>); set(linear2_kernel<192, false>); set(linear2_kernel<256, false>);
-  set(linear2_kernel<128, true>); set(linear2_kernel<192, true>); set(linear2_kernel<256, true>);
+  set(linear2_kernel<128, false>); set(linear2_kernel<256, false>);
+  set(linear2_kernel<128, true>); set(linear2_kernel<256, true>);
   return e;
 }
 
@@ -392,7 +390,6 @@ cudaError_t launch_linear_pair(const CUtensorMap& a_hi, const CUtensorMap& a_lo,
     return cudaErrorInvalidValue;
   }
   if (block_n == 256) return launch_impl2<256>(a_hi, a_lo, w_hi, w_lo, p, num_sms, stream, st);
-  if (block_n == 192) return launch_impl2<192>(a_hi, a_lo, w_hi, w_lo, p, num_sms, stream, st);
   if (block_n == 128) return launch_impl2<128>(a_hi, a_lo, w_hi, w_lo, p, num_sms, stream, st);
   set_last_error("launch_linear_pair: unsupported block_n %d", block_n);
   return cudaErrorInvalidValue;

@@ -199,25 +199,25 @@ __device__ __forceinline__ float pick(const float (&a)[kSlicesPerWarp], int k) {
 }
 
 // Start of a tile for one epilogue warp: per-column constants of its (up to) four 32-column slices and the statistics of
-// its row.  `wide`: the warp owns two 64-column pairs (slices 2q, 2q+1 for q = warp_in_group, warp_in_group + 2) instead
-// of the alternating slices warp_in_group + 2k.
-__device__ __forceinline__ int warp_slice(int k, int warp_in_group, bool wide) {
-  return wide ? 2 * (warp_in_group + kWarpsPerLaneGroup * (k >> 1)) + (k & 1) : warp_in_group + k * kWarpsPerLaneGroup;
+// its row.  `pairs` (ChainPhaseInfo::pair_epilogue): the warp owns two 64-column pairs (slices 2q, 2q+1 for
+// q = warp_in_group, warp_in_group + 2) instead of the alternating slices warp_in_group + 2k.
+__device__ __forceinline__ int warp_slice(int k, int warp_in_group, bool pairs) {
+  return pairs ? 2 * (warp_in_group + kWarpsPerLaneGroup * (k >> 1)) + (k & 1) : warp_in_group + k * kWarpsPerLaneGroup;
 }
 // The constants do not depend on anything computed in this launch: they are requested BEFORE the warp waits for the tile's
 // accumulator, all loads of a vector in flight together (indices clamped instead of predicated; measured before: one
 // predicated load at a time, each followed by the spill of its result, was 11 % of this kernel's stall samples).
-__device__ __forceinline__ void load_tile_constants(const LinearParams& p, RowStats& rs, int n_blk, int warp_in_group, bool wide, int lane) {
+__device__ __forceinline__ void load_tile_constants(const LinearParams& p, RowStats& rs, int n_blk, int warp_in_group, bool pairs, int lane) {
   int idx[kSlicesPerWarp];
   bool ok[kSlicesPerWarp];
 #pragma unroll
   for (int k = 0; k < kSlicesPerWarp; ++k) {
-    const int sl = warp_slice(k, warp_in_group, wide);
+    const int sl = warp_slice(k, warp_in_group, pairs);
     const int n = n_blk * kBlockN + sl * 32 + lane;
     ok[k] = sl < kSlices && n < p.N;
     idx[k] = ok[k] ? n : 0;
   }
-  const bool ln = p.ln_src || p.ln_src_hi;
+  const bool ln = p.ln_src_hi != nullptr;
   float t[4][kSlicesPerWarp];
 #pragma unroll
   for (int k = 0; k < kSlicesPerWarp; ++k) {
@@ -297,7 +297,7 @@ __device__ __forceinline__ void epilogue_pair(const LinearParams& p, const Chain
 }
 
 // One 32-column slice of a 128-row accumulator: TMEM -> registers -> [folded LayerNorm] -> bias -> [residual] ->
-// [partial statistics] -> [GELU] -> fp32 rows and/or bf16 hi/lo planes.
+// [partial statistics] -> row-mapped fp32 rows (output head) or bf16 hi/lo planes.
 __device__ __forceinline__ void epilogue_slice(const LinearParams& p, const ChainPhaseDesc& pd, uint32_t tmem_acc, int m_blk, int n_blk,
                                                int slice, int k_in_tile, int lane_group, int lane, uint32_t stage, RowStats& rs, uint4 (&rv)[8],
                                                bool& rv_ready, int next_slice, int warp_in_group, long long* dbg) {
@@ -307,15 +307,14 @@ __device__ __forceinline__ void epilogue_slice(const LinearParams& p, const Chai
   const int row = warp_row0 + lane;
   const int n0 = n_blk * kBlockN + slice * 32;
   if (n0 >= p.N) return;  // warp-uniform: columns beyond the layer's width (output head)
-  const float* res_src = p.residual ? p.residual : p.ln_src;
-  const bool res_planes = p.ln_src_hi != nullptr;  // LayerNorm's input as bf16 hi / lo planes instead of fp32 rows
-  const bool has_res = res_src || res_planes;
+  // residual = LayerNorm(v) re-derived from v's bf16 hi / lo planes, or fp32 rows added as they are (layer 0's out-proj)
+  const bool res_planes = p.ln_src_hi != nullptr;
+  const bool has_res = p.residual || res_planes;
   // the staging tile is about to be rewritten (residual fetch or stores): the bulk store issued from it has been read out
   CMDI_T(8);   // row statistics
   if (lane == 0) tma_store_wait_read();
   __syncwarp();
   CMDI_T(9);   // staging free
-  const long long res_ld = p.residual ? p.ld_res : p.ld_ln;
   // Residual block of 32 rows x 32 columns, fetched coalesced into rv: fp32 rows (8 x 16 B per thread, 4 complete 128 B
   // row segments per instruction) or the two bf16 planes (4 + 4 x 16 B, 8 complete 64 B segments per instruction).
   // Under this kernel's load an L2 round trip costs ~2 us, so the block of the warp's NEXT slice of the same tile is
@@ -331,7 +330,7 @@ __device__ __forceinline__ void epilogue_slice(const LinearParams& p, const Chai
     } else {
 #pragma unroll
       for (int it = 0; it < 8; ++it)
-        rv[it] = ld_global_cg_v4(res_src + (long long)(warp_row0 + it * 4 + (lane >> 3)) * res_ld + n + (lane & 7) * 4);
+        rv[it] = ld_global_cg_v4(p.residual + (long long)(warp_row0 + it * 4 + (lane >> 3)) * p.ld_res + n + (lane & 7) * 4);
     }
   };
   if (has_res && !rv_ready) fetch_residual(n0);
@@ -400,16 +399,8 @@ __device__ __forceinline__ void epilogue_slice(const LinearParams& p, const Chai
 #pragma unroll
       for (int g = 0; g < 8; ++g) {
         const uint4 u = ld_shared_v4(stage + lane * 128 + ((g ^ (lane & 7)) << 4));
-        if (p.ln_src) {
-          // residual = LayerNorm(ln_src) re-derived from its fp32 input, the row statistics and gamma / beta
-          f[g * 4 + 0] += ln_apply(__uint_as_float(u.x), rs.ln.x, rs.ln.y, __shfl_sync(0xffffffffu, gk, g * 4 + 0), __shfl_sync(0xffffffffu, btk, g * 4 + 0));
-          f[g * 4 + 1] += ln_apply(__uint_as_float(u.y), rs.ln.x, rs.ln.y, __shfl_sync(0xffffffffu, gk, g * 4 + 1), __shfl_sync(0xffffffffu, btk, g * 4 + 1));
-          f[g * 4 + 2] += ln_apply(__uint_as_float(u.z), rs.ln.x, rs.ln.y, __shfl_sync(0xffffffffu, gk, g * 4 + 2), __shfl_sync(0xffffffffu, btk, g * 4 + 2));
-          f[g * 4 + 3] += ln_apply(__uint_as_float(u.w), rs.ln.x, rs.ln.y, __shfl_sync(0xffffffffu, gk, g * 4 + 3), __shfl_sync(0xffffffffu, btk, g * 4 + 3));
-        } else {
-          f[g * 4 + 0] += __uint_as_float(u.x); f[g * 4 + 1] += __uint_as_float(u.y);
-          f[g * 4 + 2] += __uint_as_float(u.z); f[g * 4 + 3] += __uint_as_float(u.w);
-        }
+        f[g * 4 + 0] += __uint_as_float(u.x); f[g * 4 + 1] += __uint_as_float(u.y);
+        f[g * 4 + 2] += __uint_as_float(u.z); f[g * 4 + 3] += __uint_as_float(u.w);
       }
     }
   }
@@ -436,30 +427,22 @@ __device__ __forceinline__ void epilogue_slice(const LinearParams& p, const Chai
     if (k_in_tile == kSlicesPerWarp - 1)
       p.stats_out[(size_t)row * kPartialStride + n_blk * kWarpsPerLaneGroup + warp_in_group] = make_float2(rs.run_mean, rs.run_m2);
   }
-  if (p.act == 1) {
-#pragma unroll
-    for (int j = 0; j < 32; ++j) f[j] = gelu_fast(f[j]);
-  }
-  CMDI_T(12);  // statistics + activation
+  CMDI_T(12);  // statistics
   if (p.out_f32) {
+    // row-mapped fp32 output (output head: sequence rows -> frame rows, token row dropped): masked coalesced stores
     uint32_t w[32];
 #pragma unroll
     for (int j = 0; j < 32; ++j) w[j] = __float_as_uint(f[j]);
-    if (p.tma_store) {
-      store_block_tma(stage, lane, w, &pd.o_f32, n0, warp_row0);
-    } else {
-      // row-mapped fp32 output (output head: sequence rows -> frame rows, token row dropped): masked coalesced stores
-      RowSlots rows;
-      rows.ok = 0;
+    RowSlots rows;
+    rows.ok = 0;
 #pragma unroll
-      for (int it = 0; it < 8; ++it) {
-        int pos_unused;
-        long long r;
-        if (map_row(p, warp_row0 + it * 4 + (lane >> 3), r, pos_unused)) rows.ok |= 1u << it;
-        rows.row[it] = (int)r;
-      }
-      store_block_coalesced(stage, lane, w, reinterpret_cast<char*>(p.out_f32 + n0), rows, (long long)p.ld_f32 * 4, (p.N - n0) / 4, 1, 0);
+    for (int it = 0; it < 8; ++it) {
+      int pos_unused;
+      long long r;
+      if (map_row(p, warp_row0 + it * 4 + (lane >> 3), r, pos_unused)) rows.ok |= 1u << it;
+      rows.row[it] = (int)r;
     }
+    store_block_coalesced(stage, lane, w, reinterpret_cast<char*>(p.out_f32 + n0), rows, (long long)p.ld_f32 * 4, (p.N - n0) / 4, 1, 0);
   }
   CMDI_T(13);  // fp32 store
   if (p.out_hi) {
@@ -661,7 +644,7 @@ linear_chain_kernel(const ChainPhaseDesc* __restrict__ phases, const int num_pha
     const int j3 = ew >> 2;               // index within the lane group
     const uint32_t epi_stage_addr = smem_u32(epi_stage + ew * kEpiStageBytes);
     const uint32_t tmem_lane = tmem_base + ((uint32_t)(lane_group * 32) << 16);
-    int ph = 0, stored_seq = -1;
+    int ph = 0;
     RowStats rs{};
     // everything this warp stored for tile `seq` is in memory: tell the publisher
     auto publish = [&](int seq) {
@@ -680,20 +663,15 @@ linear_chain_kernel(const ChainPhaseDesc* __restrict__ phases, const int num_pha
       const int m_blk = 2 * (local / pi.num_n_blocks) + (int)cta_rank;
       const int n_blk = local % pi.num_n_blocks;
       const int acc = seq & 1;
-      const bool wide = pi.wide != 0;
-      load_tile_constants(pi.p, rs, n_blk, j3, wide, lane);
+      const bool pairs = pi.pair_epilogue != 0;
+      load_tile_constants(pi.p, rs, n_blk, j3, pairs, lane);
       mbar_wait(&bars->tmem_full[acc], (seq >> 1) & 1);
       long long c1 = clock64();
       tc_fence_after();
-      if (stored_seq >= 0) {
-        publish(stored_seq);  // deferred from the previous tile: its stores have landed while the mainloop ran
-        stored_seq = -1;
-      }
-      long long c2 = clock64();
       load_row_statistics(pi.p, rs, m_blk * kBlockM + lane_group * 32 + lane);
       const uint32_t tmem_acc = tmem_lane + acc * kAccStride;
       long long* dbg_w = (dbg_me && ew == 0 && lane == 0) ? dbg_me + ph * 16 : nullptr;
-      if (wide) {
+      if (pairs) {
 #pragma unroll 1
         for (int k2 = 0; k2 < kSlicesPerWarp / 2; ++k2) {
           epilogue_pair(pi.p, phases[ph], tmem_acc, m_blk, n_blk, j3 + kWarpsPerLaneGroup * k2, k2, lane_group, lane, epi_stage_addr, rs);
@@ -718,22 +696,12 @@ linear_chain_kernel(const ChainPhaseDesc* __restrict__ phases, const int num_pha
           if (lane == 0) mbar_arrive_on_leader(&bars->tmem_empty[acc]);
         }
       }
-      stored_seq = seq;
-      long long c3 = clock64();
-      {
-        // If this cluster's next tile belongs to a later phase (or does not exist) it may depend on this one: publish
-        // now; otherwise at the start of the next tile.
-        const int next_tile = cluster_id + (seq + 1) * num_clusters;
-        if (next_tile >= pi.tile_end || pi.publish_now) {
-          publish(seq);
-          stored_seq = -1;
-        }
-      }
+      long long c2 = clock64();
+      publish(seq);
       if (dbg_me && ew == 0 && lane == 0) {
-        dbg_me[ph * 16 + 5] += c1 - c0; dbg_me[ph * 16 + 6] += c3 - c2; dbg_me[ph * 16 + 7] += (c2 - c1) + (clock64() - c3);
+        dbg_me[ph * 16 + 5] += c1 - c0; dbg_me[ph * 16 + 6] += c2 - c1; dbg_me[ph * 16 + 7] += clock64() - c2;
       }
     }
-    if (stored_seq >= 0) publish(stored_seq);
     if (lane == 0) tma_store_wait_all();
   }
 

@@ -164,10 +164,9 @@ template <int BLOCK_N>
 __device__ __forceinline__ void epilogue_tile(const LinearParams& p, const EpiStoreMaps& maps, uint32_t tmem_base, uint32_t acc_col,
                                               int m_blk, int n_blk, int lane_group, int col_part, int lane, uint32_t stage) {
   constexpr int kBlockM = kEpiBlockM;
-  // the two column parts of a tile: halves, except BLOCK_N = 192 -> 128 + 64 (whole 64-column chunks per warp)
-  constexpr int kPart0Cols = (BLOCK_N == 192) ? 128 : BLOCK_N / 2;
-  const int col_start = col_part == 0 ? 0 : kPart0Cols;
-  const int part_cols = col_part == 0 ? kPart0Cols : BLOCK_N - kPart0Cols;
+  // the two column parts of a tile: halves (whole 64-column chunks per warp)
+  constexpr int part_cols = BLOCK_N / 2;
+  const int col_start = col_part == 0 ? 0 : part_cols;
   const int warp_row0 = m_blk * kBlockM + lane_group * 32;
   RowSlots rows;
   rows.ok = 0;

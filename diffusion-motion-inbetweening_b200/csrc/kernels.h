@@ -52,7 +52,7 @@ struct LinearParams {
   const float2* ln_partials;
   // ... with LayerNorm's input read back as the bf16 hi + lo planes [rows, ld_ln] the producer wrote for the next GEMM
   // anyway (v = hi + lo to 2^-17 relative: the same quantisation the GEMMs' A operand already has), so that the
-  // producer need not store an fp32 copy as well.  Takes precedence over ln_src.
+  // producer need not store an fp32 copy as well.  The chained epilogue reads LayerNorm's input only this way (not ln_src).
   const __nv_bfloat16* ln_src_hi;
   const __nv_bfloat16* ln_src_lo;
   // LayerNorm folded into THIS linear layer (the A operand is the un-normalised v, the W operand is W * gamma):
@@ -111,11 +111,12 @@ struct ChainPhaseInfo {
   int* wait_ctr;               // [num_m_pairs] or null: A rows of pair m are complete when wait_ctr[m] >= wait_target
   int wait_target;
   int* done_ctr;               // [num_m_pairs] or null: each CTA adds 1 once its half of a tile is in memory
-  int publish_now;             // 1: bump done_ctr as soon as a tile's stores have landed (the warp waits for them); 0: at its next tile
-  int wide;                    // 1: planes-only phase whose epilogue works on 64-column pairs (o_hi / o_lo are {64, 32} boxes, 128 B swizzle)
+  // 1: planes-only phase (FFN1, QKV) whose epilogue works on 64-column pairs, o_hi / o_lo are {64, 32} boxes with the
+  // 128 B swizzle;  0: 32-column slices (residual phases, output head), o_hi / o_lo are {32, 32} boxes with the 64 B swizzle
+  int pair_epilogue;
 };
 struct alignas(128) ChainPhaseDesc {
-  CUtensorMap a_hi, a_lo, w_hi, w_lo, o_hi, o_lo, o_f32;
+  CUtensorMap a_hi, a_lo, w_hi, w_lo, o_hi, o_lo;
   ChainPhaseInfo info;
 };
 cudaError_t configure_linear_chain_kernel();
@@ -137,7 +138,6 @@ struct AttnParams {
   __nv_bfloat16* out_lo;
   int ld_out;
   long long* dbg_cycles;  // bring-up only: [num_clusters][16] cycle counters or null
-  int trunc_split;        // 1: hi plane of P and O by truncation (split_bf16x2_trunc): half the conversions, error 2^-16 instead of 2^-17
 };
 // qkv maps: bf16 [rows, 3*H*128] row-major planes (hi, lo); box {64, 128} for Q, {64, 208} for V (and K in the backward
 // kernel), {64, 104} for K (each CTA of a pair holds half of the keys).

@@ -48,8 +48,8 @@ def run_linear(M, N, K, prec, bn, act=0, bias=True, res=False, seed=0, scale=1.0
     (12608, 1536, 512, 256), (12544, 512, 263, 128), (12608, 264, 512, 128), (25216, 512, 1024, 128),
     # negative block_n: the CTA-pair kernel (cta_group::2), tile 256 x |block_n|
     (256, 256, 64, -256), (1, 8, 8, -128), (130, 264, 512, -128), (1000, 1536, 512, -256), (12608, 1536, 512, -256),
-    (12608, 512, 1024, -128), (256, 192, 64, -192), (1000, 1536, 512, -192), (12608, 1536, 512, -192), (300, 1000, 512, -192),
-    (25216, 1536, 512, -192),
+    (12608, 512, 1024, -128), (256, 192, 64, -128), (1000, 1536, 512, -128), (12608, 1536, 512, -128), (300, 1000, 512, -256),
+    (25216, 1536, 512, -256),
 ])
 def test_linear_bf16x3_meets_fp32_gate(M, N, K, bn):
     out, ref = run_linear(M, N, K, 3, bn)
@@ -58,7 +58,7 @@ def test_linear_bf16x3_meets_fp32_gate(M, N, K, bn):
     assert (out - ref).abs().max() < 1e-4  # typical 3e-5 at |C| ~ 7
 
 
-@pytest.mark.parametrize("bn", [256, -256, -192, -128])
+@pytest.mark.parametrize("bn", [256, -256, -128])
 @pytest.mark.parametrize("act,res", [(1, False), (0, True), (1, True)])
 def test_linear_epilogues(act, res, bn):
     out, ref = run_linear(777, 1024, 512, 3, bn, act=act, res=res)

@@ -55,6 +55,37 @@ def test_product_never_imports_the_oracle():
             assert "oracle" not in src.replace("no CPU fallback", ""), fn
 
 
+def test_environment_switches_are_read_only_at_engine_creation():
+    """Engine state is per handle (DESIGN.md 1): the library reads the environment only inside cmdi_engine_create, and the
+    switches of the variants that lost their A/B measurements stay removed.  The test harness capi_test.cu is exempt
+    from the first rule."""
+    csrc = os.path.join(ROOT, "diffusion-motion-inbetweening_b200", "csrc")
+    # spelled without the prefix, so that searching the repository for a removed switch finds only its history in profiles/
+    removed = ["CMDI_" + s for s in ("CHAIN_RES", "CHAIN_WIDE", "CHAIN_PUBLISH", "EPI", "BN_QKV", "BN_WIDE", "BN_NARROW",
+                                     "ATTN_SPLIT", "GRAPH_STEPS", "CONV_REUSE")]
+    code_only = re.compile(r'//[^\n]*|/\*.*?\*/|"(?:\\.|[^"\\\n])*"|\'(?:\\.|[^\'\\\n])*\'', re.S)
+    sources = sorted(fn for fn in os.listdir(csrc) if fn.endswith((".cu", ".cuh", ".inc", ".h")))
+    assert "engine.cu" in sources and "gemm2.cu" in sources
+    for fn in sources:
+        src = open(os.path.join(csrc, fn)).read()
+        for name in removed:
+            assert not re.search(rf"\b{name}\b", src), f"{fn} still names {name}"
+        if fn == "capi_test.cu":
+            continue
+        code = code_only.sub(lambda m: " " * len(m.group(0)), src)  # same offsets, no braces or calls in comments / strings
+        allowed = range(0)
+        if fn == "engine.cu":
+            start = re.search(r"\bcmdi_engine_create\s*\([^;{]*\)\s*\{", code).end() - 1
+            depth, end = 0, start
+            for end in range(start, len(code)):
+                depth += {"{": 1, "}": -1}.get(code[end], 0)
+                if depth == 0:
+                    break
+            allowed = range(start, end)
+        for m in re.finditer(r"\bgetenv\s*\(", code):
+            assert m.start() in allowed, f"{fn}:{code.count(chr(10), 0, m.start()) + 1}: getenv outside cmdi_engine_create"
+
+
 @pytest.mark.parametrize("resp", ["", "ddim50", "ddim100", "10,15,20"])
 def test_diffusion_tables_equal_reference(golden_dir, resp):
     g = np.load(os.path.join(golden_dir, "schedules.npz"))
